@@ -141,6 +141,28 @@ def host_queries(n: int) -> np.ndarray:
     return (q / np.linalg.norm(q, axis=1, keepdims=True)).astype(np.float32)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays: dict) -> None:
+    """--dump-outputs: write what the timed calls returned in their last step as DIR/<name>.npy (ids as float64, exact
+    below 2**53; scores as float32), so that two builds can be compared output for output on the same seeded inputs."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    conv = {name: np.ascontiguousarray(a, dtype=np.float32 if np.asarray(a).dtype == np.float32 else np.float64)
+            for name, a in arrays.items()}
+    total = sum(a.nbytes for a in conv.values())
+    assert total <= DUMP_LIMIT_BYTES, f"dump of {total} bytes exceeds {DUMP_LIMIT_BYTES}"
+    for name, a in conv.items():
+        np.save(out / f"{name}.npy", a)
+
+
+def result_arrays(prefix: str, result) -> dict:
+    """One search result (a list of (frame_id, score) pairs) as the arrays dump_outputs writes."""
+    return {f"{prefix}_ids": np.array([r[0] for r in result], np.float64),
+            f"{prefix}_scores": np.array([r[1] for r in result], np.float32)}
+
+
 def host_mem_available_gb() -> float:
     try:
         for line in Path("/proc/meminfo").read_text().splitlines():
@@ -321,22 +343,25 @@ def run_single(args):
         "clocks": clocks,
         "check": {"top1_frame_id": last[0][0] if last else None, "top1_score": last[0][1] if last else None},
     }
+    outputs = result_arrays("e2e", last) if last else {}
     if not args.no_shadow and not small:
         try:                        # an extra measurement must never cost the headline line
-            line["shadow_filtered"] = shadow_filtered_arm(eng, args, qs, n_distinct)
+            line["shadow_filtered"] = shadow_filtered_arm(eng, args, qs, n_distinct, outputs)
         except Exception as ex:     # noqa: BLE001
             line["shadow_filtered"] = {"error": repr(ex)}
     if not args.no_shadow and not small:
         try:                        # BASELINE configs[2] on the same resident corpus: the tensor-bound companion number
-            line["batched"] = batched_arm(eng, args)
+            line["batched"] = batched_arm(eng, args, outputs=outputs)
         except Exception as ex:     # noqa: BLE001
             line["batched"] = {"error": repr(ex)}
     if not args.no_shadow and not small:
         eng.close()                 # free the 23 GB of configs[1]/[2] before the 46 GB of configs[4]
         try:
-            line["batched_c5"] = batched_c5_arm()
+            line["batched_c5"] = batched_c5_arm(outputs=outputs)
         except Exception as ex:     # noqa: BLE001
             line["batched_c5"] = {"error": repr(ex)}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     if not args.no_cpu_baseline:
         base = cpu_reference_arm(args.rows, steps=5, warmup=1, budget_s=20.0)
         line["cpu_baseline"] = {k: base[k] for k in ("value", "unit", "cores", "kind", "sample")}
@@ -355,9 +380,10 @@ def _tensor_peaks():
         return {}
 
 
-def _batched_line(eng, rows, dims, batch, top_k, metric_name, workload, steps):
+def _batched_line(eng, rows, dims, batch, top_k, metric_name, workload, steps, outputs=None, name=""):
     """Device-only time (CUDA events inside the library) + the same batch END TO END through wax_vs_search_batch with
-    HOST buffers (queries H2D, ids/scores D2H inside the timed region) + which level answered."""
+    HOST buffers (queries H2D, ids/scores D2H inside the timed region) + which level answered.  The arrays of the last
+    end-to-end step go into `outputs` (a dict) as <name>_ids / _scores / _counts when it is given."""
     import torch
     peaks = _tensor_peaks()
     ms, launches, unproven = eng.time_search_batch(batch, top_k, steps, warmup=4, seed=QUERY_SEED)
@@ -378,6 +404,8 @@ def _batched_line(eng, rows, dims, batch, top_k, metric_name, workload, steps):
         ids, scores, ns = eng.search_batch_arrays(qs, top_k)
     torch.cuda.synchronize()
     e2e_s = (time.perf_counter() - t0) / steps
+    if outputs is not None:
+        outputs.update({f"{name}_ids": ids, f"{name}_scores": scores, f"{name}_counts": ns})
     t1q, f1q = eng.batch_stats()
     return {
         "workload": workload, "value": batch / per * 1e3, "unit": "queries/s", "ms_per_step": per, "steps": steps,
@@ -399,15 +427,17 @@ def _batched_line(eng, rows, dims, batch, top_k, metric_name, workload, steps):
     }
 
 
-def batched_arm(eng, args, batch: int = 1024, steps: int = 10):
+def batched_arm(eng, args, batch: int = 1024, steps: int = 10, outputs=None):
     """NOT the headline: BASELINE configs[2] (batch of 1024 queries, top-10 cosine) on the corpus already resident for
     the headline -- tcgen05 nominations over the bf16 shadow + exact fp32 re-score + completeness proof (DESIGN 4.5.1),
     results identical to 1024 single-query scans (tests/test_gpu_fullsize.py checks that at this size)."""
     return _batched_line(eng, args.rows, DIMS, batch, TOP_K, "queries/sec cosine top-10, batch 1024 @ 10Mx384 fp32",
-                         f"{args.rows} x {DIMS} fp32 corpus (BASELINE configs[2]), batch {batch}, top-{TOP_K} cosine", steps)
+                         f"{args.rows} x {DIMS} fp32 corpus (BASELINE configs[2]), batch {batch}, top-{TOP_K} cosine", steps,
+                         outputs, "batched")
 
 
-def batched_c5_arm(rows: int = 10_000_000, dims: int = 768, batch: int = 256, top_k: int = 100, steps: int = 10):
+def batched_c5_arm(rows: int = 10_000_000, dims: int = 768, batch: int = 256, top_k: int = 100, steps: int = 10,
+                   outputs=None):
     """NOT the headline: BASELINE configs[4] -- 10 M x 768 fp32 rows that are NOT normalised, batch 256, top-100 under
     the dot metric (score = q.v - 1).  Its own engine (30.7 GB corpus + 15.4 GB bf16 shadow)."""
     from wax_b200 import CUDAVectorEngine, VectorMetric
@@ -415,12 +445,13 @@ def batched_c5_arm(rows: int = 10_000_000, dims: int = 768, batch: int = 256, to
     try:
         eng.fill_synthetic(5, rows, normalize=False)
         return _batched_line(eng, rows, dims, batch, top_k, "queries/sec dot top-100, batch 256 @ 10Mx768 fp32",
-                             f"{rows} x {dims} fp32 un-normalised corpus (BASELINE configs[4]), batch {batch}, top-{top_k} dot", steps)
+                             f"{rows} x {dims} fp32 un-normalised corpus (BASELINE configs[4]), batch {batch}, top-{top_k} dot", steps,
+                             outputs, "batched_c5")
     finally:
         eng.close()
 
 
-def shadow_filtered_arm(eng, args, qs, n_distinct):
+def shadow_filtered_arm(eng, args, qs, n_distinct, outputs=None):
     """NOT the headline (`value` / `e2e` above are the fused fp32 scan north_star names): the same single-query
     workload with the opt-in `single_shadow` mode -- the query is first ranked against the bf16 shadow of the corpus
     (half the HBM bytes, DESIGN 4.5.1), the best nominees are re-scored exactly in fp32 and a completeness proof
@@ -439,6 +470,8 @@ def shadow_filtered_arm(eng, args, qs, n_distinct):
         torch.cuda.synchronize()
         e2e_s = time.perf_counter() - t0
         same = all(got[i] == expect[i % len(expect)] for i in range(args.steps))
+        if outputs is not None and got:
+            outputs.update(result_arrays("shadow_filtered", got[-1]))
         return {
             "value": args.steps / (ms / 1e3), "unit": "queries/s", "ms_per_step": ms / args.steps,
             "e2e": {"value": args.steps / e2e_s, "unit": "queries/s", "ms_per_step": e2e_s / args.steps * 1e3},
@@ -560,6 +593,8 @@ def run_sharded(args, rank: int, world: int, local_rank: int):
         }
         if weak is not None:
             line["weak"] = weak
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, result_arrays("e2e", last))
         print(json.dumps(line), flush=True)
     dist.destroy_process_group()
 
@@ -604,6 +639,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-shadow", action="store_true", help="skip the extra `shadow_filtered` (opt-in mode) measurement")
     ap.add_argument("--no-weak", action="store_true", help="N>1: skip the extra weak-scaling (12.5 M rows per GPU) measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the results of the last timed step of each search measured "
+                         "(e2e_*: the public single-query search; batched_*, batched_c5_*, shadow_filtered_*: the extra "
+                         "arms that ran) as DIR/<name>.npy; the inputs are seeded, so two builds compare output for output")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
